@@ -8,6 +8,7 @@ Metric = audio-seconds of window audio processed per wall second (RTF^-1), whole
   python bench.py --gpus 1 --steps 10 --warmup 3
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference         # the reference algorithm on the host cores (oracle port)
+  python bench.py --dump-outputs DIR       # also write the last timed step's outputs as DIR/*.npy (to compare builds)
 """
 from __future__ import annotations
 
@@ -23,6 +24,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 SR = 16000
@@ -160,8 +162,10 @@ def run_reference(args):
         seg_forward(a, sd, wav[:max(1, per_step // 4)])
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        seg_forward(a, sd, wav)
+        logp = seg_forward(a, sd, wav)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logp": logp})
     val = args.steps * per_step * N / SR / dt
     sample = f"{per_step} windows x {args.seconds:g} s per step ({args.steps} steps), fp32 torch oracle port of Model.forward"
     out = {
@@ -193,15 +197,18 @@ def run_reference_pipeline(args):
     masks = torch.ones(nw, 1, T)
 
     def step():
-        seg_forward(a, sd, wav)
+        logp = seg_forward(a, sd, wav)
         for _ in range(4):
-            emb_forward(esd, wav, masks)
+            emb = emb_forward(esd, wav, masks)
+        return logp, emb
     for _ in range(max(1, args.warmup)):
         seg_forward(a, sd, wav[:1]); emb_forward(esd, wav[:1], masks[:1])
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        logp, emb = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logp": logp, "embeddings": emb})
     val = args.steps * nw * dur * 0.1 / dt
     sample = (f"{nw} windows x {dur:g} s per step ({args.steps} steps): oracle port of Model.forward + 4 ResNet34 passes per window "
               f"(trunk per (window, speaker) pair); stream seconds = windows x {dur * 0.1:g} s step; clustering excluded")
@@ -422,6 +429,10 @@ def run_pipeline_bench(args, world, rank, local, dist):
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        res = pipe.last             # the dict the last timed diarize_waveform call returned; `ann` is its Annotation
+        dump_outputs(args.dump_outputs, {"turns": turns(ann), **{k: res[k] for k in (
+            "segmentations", "count", "embeddings", "hard_clusters", "discrete", "centroids") if res.get(k) is not None}})
     # ---- end to end: pinned host waveform in (each rank uploads the span of its own windows), Annotation out on rank 0 ----
     one(False, sharded)
     barrier()
@@ -616,6 +627,9 @@ def run_many_bench(args, world, rank, local, dist):
         outs = pipe.diarize_many(recs, names)
     barrier()
     dt = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:      # rows of (recording, start s, end s, speaker label), the Annotations this rank returned
+        rows = [np.insert(turns(o), 0, i, axis=1) for i, o in enumerate(outs) if o is not None]
+        dump_outputs(args.dump_outputs, {"turns": np.concatenate(rows) if rows else np.zeros((0, 4))})
     done = torch.tensor([sum(o is not None for o in outs)], device="cuda")
     tt = torch.tensor([dt], device="cuda", dtype=torch.float64)
     if dist is not None:
@@ -640,19 +654,51 @@ def seg_sub_record(args):
     N, B = 5 * SR, 256
     model = SegmentationModel.random_init("wavlm_base_s80_md", seed=0, precision=args.precision)
     wav = synth_wav(B, N).cuda()
-    for _ in range(3):
+    for _ in range(args.warmup):
         model.hard(wav)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(10):
+    for _ in range(args.steps):
         model.hard(wav)
     e1.record()
     torch.cuda.synchronize()
-    ms = e0.elapsed_time(e1) / 10
+    ms = e0.elapsed_time(e1) / args.steps
     return {"workload": "wavlm_base_s80_md segmentation forward, 256 x 5 s windows per step", "ms_per_step": ms,
             "audio_s_per_s": B * 5.0 / (ms * 1e-3), "tflops": 256 * 15.2e9 / (ms * 1e-3) / 1e12,
             "frac_of_tensor_peak": 256 * 15.2e9 / (ms * 1e-3) / 1e12 / measured_peaks()["tensor"]}
+
+
+DUMP_LIMIT = 64 * 10 ** 6     # bytes, all files of one --dump-outputs directory together
+
+
+def turns(ann) -> np.ndarray:
+    """Annotation -> (turns, 3) float64 rows of start s, end s, speaker label"""
+    return np.array([(s.start, s.end, float(lab)) for s, _, lab in ann.itertracks(yield_label=True)], dtype=np.float64).reshape(-1, 3)
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: what the timed path returned in its last step, as out_dir/<name>.npy, so that two builds of the
+    project can be compared output for output on identical inputs.  float64 stays float64; float32 and integers that
+    float32 holds exactly become float32, other integers float64.  Above DUMP_LIMIT bytes in all, every array keeps the
+    same fraction of its rows (first axis), drawn with a fixed seed and kept in order; the kept row numbers then go to
+    <name>.rows.npy."""
+    conv = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        small_int = a.dtype.kind in "biu" and (a.size == 0 or int(np.abs(a.astype(np.int64)).max()) < 2 ** 24)
+        conv[name] = a.astype(np.float32 if a.dtype == np.float32 or small_int else np.float64)
+    header = 128                                          # bytes of one .npy header (numpy pads it to a multiple of 64)
+    cost = sum(a.nbytes + (8 * a.shape[0] if a.ndim else 0) for a in conv.values())   # with the row numbers
+    keep = min(1.0, (DUMP_LIMIT - 2 * header * len(conv)) / max(cost, 1))
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    for name, a in conv.items():
+        if keep < 1.0 and a.ndim and a.shape[0] > 1:
+            rows = np.sort(rng.choice(a.shape[0], max(1, int(a.shape[0] * keep)), replace=False))
+            np.save(os.path.join(out_dir, name + ".rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 _JSON_OUT = sys.stdout
@@ -679,7 +725,8 @@ def main():
     os.environ.setdefault("NCCL_DEBUG", "WARN")   # keep NCCL's version banner off stdout
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of every timed loop (default: 3 for pipeline, 5 for pipeline on N > 1, 1 for many, 10 for seg)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--recordings", type=int, default=16, help="--workload many: number of recordings in the list")
@@ -697,7 +744,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sub-records", action="store_true")
     ap.add_argument("--even-split", action="store_true", help="window-sharded mode: equal window shares (no smaller share for the clustering rank)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.workload in ("pipeline", "many"):
         args.arch = args.arch or "wavlm_large_s80_md"; args.seconds = args.seconds or 16.0; args.batch = args.batch or 32
         args.cpu_windows = args.cpu_windows or 4
@@ -705,7 +756,8 @@ def main():
         args.arch = args.arch or "wavlm_base_s80_md"; args.seconds = args.seconds or 5.0; args.batch = args.batch or 256
         args.cpu_windows = args.cpu_windows or 32
     world_env = int(os.environ.get("WORLD_SIZE", "1"))
-    args.steps = args.steps or ((5 if world_env > 1 else 3) if args.workload == "pipeline" else (1 if args.workload == "many" else 10))
+    if args.steps is None:
+        args.steps = (5 if world_env > 1 else 3) if args.workload == "pipeline" else (1 if args.workload == "many" else 10)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.impl == "reference":
@@ -762,10 +814,12 @@ def main():
     barrier()
     e0.record()
     for _ in range(args.steps):
-        model.hard(wav_dev)
+        logp, ml = model.hard(wav_dev)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"logp": logp, "multilabel": ml})
     launches = model.last_launches * args.steps
     # ---- end to end through the host entry point (pinned host buffers, H2D + D2H inside) ----
     for _ in range(2):

@@ -2,7 +2,8 @@
 
 The reference's `Model` wrapper cannot be imported (pyannote.core & co. are absent, SURVEY.md 8c), so the
 wrapper (model_wavlm_conformer.py:238-264) is re-assembled here from the importable reference parts:
-`wav2vec2_model`, `ConformerEncoder`.  Used by scripts/make_golden.py and the oracle-pinning tests.
+`wav2vec2_model`, `ConformerEncoder`.  Used by the scripts that write the golden vectors (scripts/make_golden.py,
+scripts/make_reference_golden.py).
 """
 from __future__ import annotations
 

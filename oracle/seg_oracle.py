@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY - fp32 torch restatement of the segmentation forward.
 
-Pinned (tests/test_oracle_vs_reference.py, runs where /root/reference exists) against the
-reference modules themselves and, everywhere, against tests/golden/seg_*.npz which were produced
-by scripts/make_golden.py from the *reference* modules.
+Pinned (tests/test_oracle_vs_reference.py, tests/test_golden.py) against the outputs of the reference modules
+themselves: tests/golden/reference_pins.npz and tests/golden/seg_*.npz, produced by scripts/make_reference_golden.py and
+scripts/make_golden.py from the *reference* modules.
 
 Follows:
   diarizen/models/eend/model_wavlm_conformer.py:238-264   (wrapper)

@@ -7,8 +7,8 @@ Follows
   * diarizen/clustering/VBx.py:146-178  the x-vector -> PLDA-space transform built from xvec_transform.npz / plda.npz
   * pyannote-audio/pyannote/audio/pipelines/clustering.py:601-700  VBxClustering.__call__
 
-Pinned against the reference's own VBx.py (imported from /root/reference in tests/test_oracle_vs_reference.py) and against
-tests/golden/vbx.npz (generated from it by scripts/make_golden.py).  Only tests/, __graft_entry__.smoke() and bench.py's CPU
+Pinned against the outputs of the reference's own VBx.py (tests/test_vbx.py: tests/golden/reference_pins.npz and
+tests/golden/vbx.npz, generated from it by scripts/make_reference_golden.py and scripts/make_golden.py).  Only tests/, __graft_entry__.smoke() and bench.py's CPU
 legs may import this module.
 """
 from __future__ import annotations

@@ -1,14 +1,14 @@
 """CPU: checkpoint averaging / selection (reference diarizen/ckpt_utils.py, recipes/diar_ssl/infer_avg.py) and the wav.scp
 command line (diarizen/pipelines/inference.py:194-368)."""
-import importlib.util
 import os
 
+import numpy as np
 import pytest
 import torch
 
 from diarizen_b200 import checkpoints, cli
 
-REF_CKPT = "/root/reference/diarizen/ckpt_utils.py"
+PINS = os.path.join(os.path.dirname(__file__), "golden", "reference_pins.npz")
 
 
 def _states(n=4):
@@ -28,13 +28,11 @@ def test_average_states_is_keywise_mean_and_leaves_inputs_alone():
     assert avg["bn.num_batches_tracked"].is_floating_point()   # true division, like the reference
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_CKPT), reason="reference tree not mounted")
 def test_average_states_equals_reference():
-    spec = importlib.util.spec_from_file_location("ref_ckpt_utils", REF_CKPT)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    """bit-equal to what the reference's average_states returned for _states() (reference_pins.npz)."""
+    z = np.load(PINS)
+    theirs = {f[len("average_states/"):]: torch.from_numpy(z[f]) for f in z.files if f.startswith("average_states/")}
     ours = checkpoints.average_states(_states())
-    theirs = ref.average_states(_states(), torch.device("cpu"))
     assert ours.keys() == theirs.keys()
     for k in ours:
         assert torch.equal(ours[k], theirs[k])

@@ -1,6 +1,5 @@
-"""CPU: the VBx oracle against the reference's own VBx.py (when /root/reference is mounted) and the golden fixture;
+"""CPU: the VBx oracle against the outputs of the reference's own VBx.py and the golden fixture;
 the host restatement of scipy's maxclust flat clustering against scipy."""
-import importlib.util
 import os
 
 import numpy as np
@@ -10,7 +9,7 @@ from oracle import vbx_oracle
 import vbx_util
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "vbx.npz")
-REF_VBX = "/root/reference/diarizen/clustering/VBx.py"
+PINS = os.path.join(os.path.dirname(__file__), "golden", "reference_pins.npz")
 
 
 def _case(seed=0):
@@ -36,24 +35,24 @@ def test_plda_setup_matches_golden():
     np.testing.assert_allclose(np.abs(fea), np.abs(g["fea"]), rtol=0, atol=1e-8)
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_VBX), reason="reference tree not mounted")
 @pytest.mark.parametrize("seed", [0, 1, 2])
-def test_oracle_equals_reference_vbx(seed, tmp_path):
-    spec = importlib.util.spec_from_file_location("ref_vbx", REF_VBX)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+def test_oracle_equals_reference_vbx(seed):
+    """against the reference's vbx_setup (PLDA written as vbx_util.write_plda does) and cluster_vbx on the same labels
+    (their outputs: reference_pins.npz)"""
+    z = np.load(PINS)
     xt, plda, emb, seg = _case(seed)
-    vbx_util.write_plda(str(tmp_path), seed)
     from oracle.pipeline_oracle import filter_embeddings
     train, _, _ = filter_embeddings(emb, seg)
-    x_tf, plda_tf, psi = ref.vbx_setup(str(tmp_path))
-    fea_ref = plda_tf(x_tf(train), lda_dim=128)
+    psi, fea_ref = z[f"vbx/{seed}/psi"], z[f"vbx/{seed}/fea"]
     o_x, o_p, o_psi = vbx_oracle.plda_setup(xt, plda)
-    np.testing.assert_allclose(o_psi, psi, rtol=1e-12)
-    np.testing.assert_allclose(o_p(o_x(train), lda_dim=128), fea_ref, rtol=0, atol=1e-10)
+    # two inversions and a generalized eigenproblem: their rounding follows the BLAS kernel and thread count (up to
+    # 1.5e-10 relative on psi and 3.4e-10 on the features across OpenBLAS's x86 kernels), and the stored reference
+    # values were computed with another BLAS build than the one a test run may use
+    np.testing.assert_allclose(o_psi, psi, rtol=1e-9)
+    np.testing.assert_allclose(o_p(o_x(train), lda_dim=128), fea_ref, rtol=0, atol=2e-9)
     labels = np.random.default_rng(seed).integers(0, 5, size=len(train))
     for Fa, Fb in [(0.07, 0.8), (0.3, 10.0)]:
-        g_ref, pi_ref = ref.cluster_vbx(labels, fea_ref, psi[:128], Fa=Fa, Fb=Fb, maxIters=20)
+        g_ref, pi_ref = z[f"vbx/{seed}/{Fa:g}_{Fb:g}/gamma"], z[f"vbx/{seed}/{Fa:g}_{Fb:g}/pi"]
         g, pi, _ = vbx_oracle.vb_gmm(fea_ref, psi[:128], vbx_oracle.init_responsibilities(labels), Fa, Fb, 20)
         np.testing.assert_allclose(g, g_ref, rtol=0, atol=1e-12)
         np.testing.assert_allclose(pi, pi_ref, rtol=0, atol=1e-12)
