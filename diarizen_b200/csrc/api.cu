@@ -57,6 +57,16 @@ void dz_gemm_plan_destroy(dz_gemm_plan* p) { gemm_plan_destroy(reinterpret_cast<
 int dz_layernorm(const float* x_dev, int64_t rows, int C, int ldx, const float* prescale_dev, const float* gamma_dev,
                  const float* beta_dev, int act, float* y_f32_dev, int ldy, void* y_bf_dev, int64_t bf_plane, int ldb,
                  int planes, float* mix_dev, float mix_w, int mix_src, int mix_init, int fp16, void* stream) {
+  // both kernels move rows in 16-byte float4 chunks (x, y_f32, mix) and 8-byte 16-bit chunks (y_bf), so every row
+  // start has to stay aligned; they also hold at most 1024 columns in registers
+  if (!x_dev || !gamma_dev || !beta_dev || rows < 1) return fail(DZ_ERR_INVALID, "layernorm: null pointer or no rows");
+  if (C < 1 || C > 1024) return fail(DZ_ERR_INVALID, "layernorm: C must be in [1, 1024]");
+  if (ldx < C || ldx % 4 != 0) return fail(DZ_ERR_INVALID, "layernorm: ldx must be >= C and a multiple of 4");
+  if (y_f32_dev && (ldy < C || ldy % 4 != 0)) return fail(DZ_ERR_INVALID, "layernorm: ldy must be >= C and a multiple of 4");
+  if (y_bf_dev && (ldb < C || ldb % 8 != 0 || bf_plane % 8 != 0 || (planes != 1 && planes != 2)))
+    return fail(DZ_ERR_INVALID, "layernorm: ldb must be >= C, ldb and bf_plane multiples of 8, planes 1 or 2");
+  if (act < 0 || act > 3) return fail(DZ_ERR_INVALID, "layernorm: act must be 0..3");
+  if (mix_dev && mix_src != 1 && mix_src != 2) return fail(DZ_ERR_INVALID, "layernorm: mix_src must be 1 or 2");
   LnArgs a{};
   a.x = x_dev; a.rows = rows; a.C = C; a.ldx = ldx; a.prescale = prescale_dev; a.gamma = gamma_dev; a.beta = beta_dev;
   a.act = act; a.y_f32 = y_f32_dev; a.ldy = ldy; a.y_bf = (__nv_bfloat16*)y_bf_dev; a.bf_plane = bf_plane; a.ldb = ldb;

@@ -900,11 +900,13 @@ static cudaError_t launch_bn_tma(const GemmPlan* p, cudaStream_t st) {
 }
 
 // The TMA epilogue handles: one group, no transposed output, exactly one of (fp32 | 16-bit plane) outputs, a residual of
-// the same kind as the output (or none).  Everything else takes the generic epilogue.
+// the same kind as the output (or none), and an activation after the residual only when it is ReLU (the one it applies
+// after the add).  Everything else takes the generic epilogue.
 static bool tma_epilogue_eligible(const GemmDesc& d) {
   static const bool off = (getenv("DZ_GEMM_LEGACY_EPILOGUE") != nullptr);
   if (off && d.ln_gamma == nullptr) return false;
   if (d.groups != 1 || d.out_t != nullptr) return false;
+  if (d.act_after_res && d.act != 0 && d.act != 3) return false;
   const bool f = d.out_f32 != nullptr, h = d.out_bf != nullptr;
   if (f == h) return false;
   if (f && (d.res16 != nullptr || (d.ldo % 4) != 0 || (d.residual && (d.ldr % 4) != 0))) return false;

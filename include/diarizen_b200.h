@@ -92,7 +92,8 @@ void dz_gemm_plan_destroy(dz_gemm_plan* p);
  * ---------------------------------------------------------------------------------------------- */
 /* y = act(LayerNorm(x * prescale) * gamma + beta) over the last dim C of x[rows][ldx] (eps 1e-5).
  * Outputs (each optional): fp32 y_f32[rows][ldy]; bf16 planes y_bf[planes][rows][ldb] (pad columns
- * [C, ldb) zeroed).  mix (optional): mix[rows][ldx] = (mix_init ? 0 : mix) + mix_w * (mix_src==1 ? x : y). */
+ * [C, ldb) zeroed).  mix (optional): mix[rows][ldx] = (mix_init ? 0 : mix) + mix_w * (mix_src==1 ? x : y).
+ * 1 <= C <= 1024; ldx, ldy multiples of 4 and ldb, bf_plane multiples of 8 (each >= C); DZ_ERR_INVALID otherwise. */
 int dz_layernorm(const float* x_dev, int64_t rows, int C, int ldx, const float* prescale_dev, const float* gamma_dev,
                  const float* beta_dev, int act, float* y_f32_dev, int ldy, void* y_bf_dev, int64_t bf_plane,
                  int ldb, int planes, float* mix_dev, float mix_w, int mix_src, int mix_init, int fp16, void* stream);

@@ -52,6 +52,20 @@ def _lin(x, sd, prefix):
     return F.linear(x, sd[prefix + ".weight"], sd[prefix + ".bias"])
 
 
+def conv_layer(a: SegArch, sd: Dict[str, torch.Tensor], i: int, x: torch.Tensor) -> torch.Tensor:
+    """Conv layer i of the feature extractor: (B, C_in, T_in) -> (B, C_i, T_i).  components.py:106-132."""
+    pre = "wavlm_model.feature_extractor."
+    x = F.conv1d(x, sd[f"{pre}conv_layers.{i}.conv.weight"], stride=CONV_STRIDES[i])
+    if a.large:
+        x = F.layer_norm(x.transpose(1, 2), (x.shape[1],), sd[f"{pre}conv_layers.{i}.layer_norm.weight"],
+                         sd[f"{pre}conv_layers.{i}.layer_norm.bias"]).transpose(1, 2)
+    elif i == 0:
+        C = x.shape[1]
+        x = F.group_norm(x, C, sd[f"{pre}conv_layers.0.layer_norm.weight"],
+                         sd[f"{pre}conv_layers.0.layer_norm.bias"])
+    return F.gelu(x)
+
+
 def feature_extractor(a: SegArch, sd: Dict[str, torch.Tensor], wav: torch.Tensor) -> torch.Tensor:
     """(B, N) -> (B, T, C6).  model.py:106-113 + components.py:182-209."""
     pre = "wavlm_model.feature_extractor."
@@ -59,21 +73,14 @@ def feature_extractor(a: SegArch, sd: Dict[str, torch.Tensor], wav: torch.Tensor
     if a.large:
         x = F.layer_norm(x, x.shape[-1:])
     x = x.unsqueeze(1)
-    for i, (k, s) in enumerate(zip(CONV_KERNELS, CONV_STRIDES)):
-        x = F.conv1d(x, sd[f"{pre}conv_layers.{i}.conv.weight"], stride=s)
-        if a.large:
-            x = F.layer_norm(x.transpose(1, 2), (x.shape[1],), sd[f"{pre}conv_layers.{i}.layer_norm.weight"],
-                             sd[f"{pre}conv_layers.{i}.layer_norm.bias"]).transpose(1, 2)
-        elif i == 0:
-            C = x.shape[1]
-            x = F.group_norm(x, C, sd[f"{pre}conv_layers.0.layer_norm.weight"],
-                             sd[f"{pre}conv_layers.0.layer_norm.bias"])
-        x = F.gelu(x)
+    for i in range(len(CONV_KERNELS)):
+        x = conv_layer(a, sd, i, x)
     return x.transpose(1, 2) * sd[pre + "dummy_weight"]
 
 
-def wavlm_attention(a: SegArch, sd, prefix: str, x: torch.Tensor, heads, bias: Optional[torch.Tensor]):
-    """components.py:668-725 followed by :429-486. `x` is the (possibly pre-normed) layer input."""
+def wavlm_attention_context(a: SegArch, sd, prefix: str, x: torch.Tensor, heads, bias: Optional[torch.Tensor]):
+    """components.py:668-725 followed by :429-486 up to the output projection: (B, T, h * 64) attention context of the
+    remaining heads, in their order. `x` is the (possibly pre-normed) layer input."""
     B, T, D = x.shape
     H = a.total_heads
     h = len(heads)
@@ -93,17 +100,25 @@ def wavlm_attention(a: SegArch, sd, prefix: str, x: torch.Tensor, heads, bias: O
         w = w + mask
     w = w - w.max(dim=-1, keepdim=True)[0]
     w = torch.softmax(w, dim=-1)
-    o = (w @ v).transpose(1, 2).reshape(B, T, h * HEAD_DIM)
-    return _lin(o, sd, prefix + "out_proj")
+    return (w @ v).transpose(1, 2).reshape(B, T, h * HEAD_DIM)
 
 
-def wavlm_encoder(a: SegArch, sd, feats: torch.Tensor, taps: Optional[dict] = None) -> List[torch.Tensor]:
-    """(B,T,C6) -> list of L+1 hidden states."""
-    en = "wavlm_model.encoder."
-    tr = en + "transformer."
-    x = _lin(_ln(feats, sd, en + "feature_projection.layer_norm"), sd, en + "feature_projection.projection")
-    if taps is not None:
-        taps["proj"] = x
+def wavlm_attention(a: SegArch, sd, prefix: str, x: torch.Tensor, heads, bias: Optional[torch.Tensor]):
+    """components.py:668-725 followed by :429-486. `x` is the (possibly pre-normed) layer input."""
+    return _lin(wavlm_attention_context(a, sd, prefix, x, heads, bias), sd, prefix + "out_proj")
+
+
+def encoder_bias(a: SegArch, sd, T: int) -> Optional[torch.Tensor]:
+    """Relative-position bias (H, T, T) shared by every layer; only layer 0 owns the embedding (components.py:1004-1024)."""
+    if not a.heads[0]:
+        return None
+    return position_bias(sd["wavlm_model.encoder.transformer.layers.0.attention.rel_attn_embed.weight"], T)
+
+
+def pos_conv(a: SegArch, sd, x: torch.Tensor) -> torch.Tensor:
+    """Projected features (B, T, D) -> input of layer 0: residual positional convolution (components.py:366-380), then
+    the transformer LayerNorm for post-norm models (components.py:1590-1597)."""
+    tr = "wavlm_model.encoder.transformer."
     # weight-normed grouped conv: w = g * v / ||v|| over dims (0,1) per tap  (components.py:344)
     v = sd[tr + "pos_conv_embed.conv.parametrizations.weight.original1"]
     g = sd[tr + "pos_conv_embed.conv.parametrizations.weight.original0"]
@@ -113,28 +128,41 @@ def wavlm_encoder(a: SegArch, sd, feats: torch.Tensor, taps: Optional[dict] = No
     x = x + F.gelu(pc).transpose(1, 2)
     if not a.large:   # Transformer(layer_norm_first = not encoder_layer_norm_first): components.py:1590-1597
         x = _ln(x, sd, tr + "layer_norm")
+    return x
+
+
+def wavlm_layer(a: SegArch, sd, l: int, x: torch.Tensor, bias: Optional[torch.Tensor]) -> torch.Tensor:
+    """Encoder layer l: hidden state l -> hidden state l + 1.  components.py:899-942."""
+    L = f"wavlm_model.encoder.transformer.layers.{l}."
+    heads = a.heads[l]
+    if heads:
+        xin = _ln(x, sd, L + "layer_norm") if a.large else x
+        x = x + wavlm_attention(a, sd, L + "attention.", xin, heads, bias)
+    if a.large:
+        if a.ffn[l]:
+            y = _ln(x, sd, L + "final_layer_norm")
+            y = _lin(F.gelu(_lin(y, sd, L + "feed_forward.intermediate_dense")), sd, L + "feed_forward.output_dense")
+            x = x + y
+    else:
+        x = _ln(x, sd, L + "layer_norm")
+        if a.ffn[l]:
+            y = _lin(F.gelu(_lin(x, sd, L + "feed_forward.intermediate_dense")), sd, L + "feed_forward.output_dense")
+            x = x + y
+        x = _ln(x, sd, L + "final_layer_norm")
+    return x
+
+
+def wavlm_encoder(a: SegArch, sd, feats: torch.Tensor, taps: Optional[dict] = None) -> List[torch.Tensor]:
+    """(B,T,C6) -> list of L+1 hidden states."""
+    en = "wavlm_model.encoder."
+    x = _lin(_ln(feats, sd, en + "feature_projection.layer_norm"), sd, en + "feature_projection.projection")
+    if taps is not None:
+        taps["proj"] = x
+    x = pos_conv(a, sd, x)
     ret = [x]
-    T = x.shape[1]
-    bias = None
+    bias = encoder_bias(a, sd, x.shape[1])
     for l in range(a.num_layers):
-        L = f"{tr}layers.{l}."
-        heads = a.heads[l]
-        if heads:
-            if l == 0 and bias is None:
-                bias = position_bias(sd[L + "attention.rel_attn_embed.weight"], T)
-            xin = _ln(x, sd, L + "layer_norm") if a.large else x
-            x = x + wavlm_attention(a, sd, L + "attention.", xin, heads, bias)
-        if a.large:
-            if a.ffn[l]:
-                y = _ln(x, sd, L + "final_layer_norm")
-                y = _lin(F.gelu(_lin(y, sd, L + "feed_forward.intermediate_dense")), sd, L + "feed_forward.output_dense")
-                x = x + y
-        else:
-            x = _ln(x, sd, L + "layer_norm")
-            if a.ffn[l]:
-                y = _lin(F.gelu(_lin(x, sd, L + "feed_forward.intermediate_dense")), sd, L + "feed_forward.output_dense")
-                x = x + y
-            x = _ln(x, sd, L + "final_layer_norm")
+        x = wavlm_layer(a, sd, l, x, bias)
         ret.append(x)
     return ret
 
@@ -185,14 +213,23 @@ def seg_forward(a: SegArch, sd: Dict[str, torch.Tensor], wav: torch.Tensor, taps
     if taps is not None:
         taps["reps"] = reps
     x = torch.stack(reps, dim=-1)
-    x = F.linear(x, sd["weight_sum.weight"]).squeeze(-1)
-    x = _ln(_lin(x, sd, "proj"), sd, "lnorm")
+    x = head_input(sd, F.linear(x, sd["weight_sum.weight"]).squeeze(-1))
     if taps is not None:
         taps["head_in"] = x
     for i in range(a.head_layers):
         x = conformer_block(a, sd, f"conformer.conformer_layer.{i}.", x)
     if taps is not None:
         taps["head_out"] = x
+    return classify(sd, x)
+
+
+def head_input(sd, mix: torch.Tensor) -> torch.Tensor:
+    """Weighted layer sum (B, T, D) -> conformer input (B, T, A).  model_wavlm_conformer.py:253-257."""
+    return _ln(_lin(mix, sd, "proj"), sd, "lnorm")
+
+
+def classify(sd, x: torch.Tensor) -> torch.Tensor:
+    """Last conformer block output -> powerset log-probabilities.  model_wavlm_conformer.py:258-264."""
     return torch.log_softmax(_lin(x, sd, "classifier"), dim=-1)
 
 
