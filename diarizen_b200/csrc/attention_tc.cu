@@ -3,16 +3,15 @@
 //   scores[q,k] = Q[q].K[k]  (+ gate[q] * tab[k - q + T - 1])      Q carries the 1/sqrt(64) scaling
 //   ctx[q]      = softmax_k(scores[q,:]) . V
 //
-// One CTA = 128 queries of one (window, head); keys are streamed in blocks of 64.
-//   warp 4      : TMA producer: Q tile once, then K_j (64 keys x 64 d) and V^T_j (64 d x 64 keys), 2-stage ring
-//   warp 5      : UMMA issuer: S = Q K_j^T (128x64, fp32 in TMEM), then O += P_j V_j (128x64, fp32 in TMEM)
+// One work item = 128 queries of one (window, head); keys are streamed in blocks of 64.
+//   warp 4      : TMA producer: the item's Q tile, then K_j (64 keys x 64 d) and V_j (64 keys x 64 d, or V^T_j), 3-stage ring
+//   warp 5      : UMMA issuer: S = Q K_j^T (128x64, fp32 in TMEM), then O += P_j V_j (fp32 in TMEM)
 //   warps 0..3  : softmax: one query row per thread (= one TMEM lane): tcgen05.ld S -> bias/mask -> running max with
 //                 lazy rescaling of O (tcgen05.ld/st only when the max moved by > 8 in log2 units) -> exp2 ->
 //                 bf16 P written to shared memory in the 128-byte-swizzled K-major layout the UMMA reads.
 // The reference materialises the (B*H, T, T) bias tensor and the full score matrix
 // (components.py:695-697, :455-469); here neither ever exists in HBM.
 // reference: diarizen/models/module/wav2vec2/components.py:429-486, :668-725; conformer.py:27-71 (no bias).
-#include <cstdlib>
 #include <string>
 
 #include "common.cuh"
@@ -46,189 +45,8 @@ DZ_DEVINL float ex2(float x) {
   return y;
 }
 
-__global__ void __launch_bounds__(A_THREADS, 2) attention_tc_kernel(const __grid_constant__ AttnMaps maps, const AttnArgs a) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_align1024(smem_raw);
-  uint8_t* Qs = smem;                  // 128 x 64 bf16, SW128
-  uint8_t* Ks = Qs + 16384;            // 2 x (64 keys x 64 d)
-  uint8_t* Vs = Ks + 2 * 8192;         // 2 x (64 d x 64 keys)
-  uint8_t* Ps = Vs + 2 * 8192;         // 128 x 64 bf16, SW128
-  uint64_t* bars = reinterpret_cast<uint64_t*>(Ps + 16384);
-  uint64_t* q_full = bars;
-  uint64_t* kv_full = bars + 1;   // [2]
-  uint64_t* kv_empty = bars + 3;  // [2]
-  uint64_t* s_full = bars + 5;
-  uint64_t* p_ready = bars + 6;
-  uint64_t* o_done = bars + 7;
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 8);
-  float* tab = reinterpret_cast<float*>(bars + 10);  // [2T-1 + 64 pad]
-
-  const int T = a.T;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int q0 = blockIdx.x * ABQ, hi = blockIdx.y, b = blockIdx.z;
-  const int nblk = (T + ABK - 1) / ABK;
-  const bool has_bias = a.bias_tab != nullptr;
-
-  if (threadIdx.x == 0) {
-    mbar_init(q_full, 1);
-    mbar_init(&kv_full[0], 1); mbar_init(&kv_full[1], 1);
-    mbar_init(&kv_empty[0], 1); mbar_init(&kv_empty[1], 1);
-    mbar_init(s_full, 1);
-    mbar_init(p_ready, 128);
-    mbar_init(o_done, 1);
-    mbar_fence_init();
-    tma_prefetch_desc(&maps.q); tma_prefetch_desc(&maps.k); tma_prefetch_desc(&maps.vt);
-  }
-  if (warp == 5) tmem_alloc(tmem_ptr, 128);
-  if (has_bias) {
-    const float* src = a.bias_tab + (long long)hi * (2 * T - 1);
-    for (int i = threadIdx.x; i < 2 * T - 1 + 64; i += A_THREADS) tab[i] = (i < 2 * T - 1) ? src[i] : 0.f;
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  const uint32_t tmem_S = tmem_base;        // columns [0, 64)
-  const uint32_t tmem_O = tmem_base + 64;   // columns [64, 128)
-
-  if (warp == 4) {
-    if (lane == 0) {
-      mbar_expect_tx(q_full, 16384);
-      tma_load_3d(Qs, &maps.q, q_full, a.q_col + hi * 64, q0, b);
-      for (int j = 0; j < nblk; ++j) {
-        const int s = j & 1;
-        mbar_wait(&kv_empty[s], ((j >> 1) & 1) ^ 1);
-        mbar_expect_tx(&kv_full[s], 16384);
-        tma_load_3d(Ks + s * 8192, &maps.k, &kv_full[s], a.k_col + hi * 64, j * ABK, b);
-        tma_load_3d(Vs + s * 8192, &maps.vt, &kv_full[s], j * ABK, hi * 64, b);
-      }
-    }
-  } else if (warp == 5) {
-    if (lane == 0) {
-      const uint32_t idesc = umma_idesc_bf16(128, 64, a.fp16);
-      const uint32_t qa = smem_u32(Qs), pa = smem_u32(Ps);
-      mbar_wait(q_full, 0);
-      for (int j = 0; j < nblk; ++j) {
-        const int s = j & 1;
-        mbar_wait(&kv_full[s], (j >> 1) & 1);
-        tc_fence_after();
-        const uint32_t ka = smem_u32(Ks + s * 8192), va = smem_u32(Vs + s * 8192);
-        // S = Q K^T   (safe to overwrite S: p_ready of block j-1 was observed before PV_{j-1} was issued)
-#pragma unroll
-        for (int k = 0; k < 4; ++k) umma_bf16(tmem_S, umma_desc_sw128(qa + k * 32), umma_desc_sw128(ka + k * 32), idesc, k > 0);
-        umma_commit(s_full);
-        // O += P V
-        mbar_wait(p_ready, j & 1);
-        tc_fence_after();
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-          umma_bf16(tmem_O, umma_desc_sw128(pa + k * 32), umma_desc_sw128(va + k * 32), idesc, (j > 0 || k > 0) ? 1u : 0u);
-        umma_commit(&kv_empty[s]);
-      }
-      umma_commit(o_done);
-    }
-  } else {
-    // ---------------- softmax warps: thread <-> query row <-> TMEM lane ----------------
-    const int row = threadIdx.x;  // 0..127
-    const int tq = q0 + row;
-    const bool qvalid = tq < T;
-    const uint32_t lane_off = (uint32_t)(warp * 32) << 16;
-    const float gate = (has_bias && a.gate != nullptr) ? a.gate[((long long)b * a.nheads + hi) * T + (qvalid ? tq : T - 1)] * LOG2E : 0.f;
-    const float* trow = tab + (T - 1) - (qvalid ? tq : T - 1);  // trow[k] = tab[k - q + T - 1]
-    float m_used = -INFINITY, lsum = 0.f;
-    uint8_t* prow = Ps + row * 128;
-    const int sw = row & 7;
-    for (int j = 0; j < nblk; ++j) {
-      mbar_wait(s_full, j & 1);
-      tc_fence_after();
-      uint32_t r[64];
-      tmem_ld_32x32(tmem_S + lane_off, r);
-      tmem_ld_32x32(tmem_S + lane_off + 32, r + 32);
-      tmem_ld_wait();
-      const int kbase = j * ABK;
-      float mx = -INFINITY;
-#pragma unroll
-      for (int c = 0; c < 64; ++c) {
-        float s2 = __uint_as_float(r[c]) * LOG2E;
-        if (has_bias) s2 = fmaf(gate, trow[kbase + c], s2);
-        s2 = (kbase + c < T) ? s2 : -INFINITY;
-        r[c] = __float_as_uint(s2);
-        mx = fmaxf(mx, s2);
-      }
-      // lazy rescale: keep exponentials relative to m_used unless the row maximum moved by more than 2^8
-      const bool need = mx > m_used + 8.0f;
-      float corr = 1.0f;
-      if (need) {
-        corr = ex2(m_used - mx);  // 0 on the first block (m_used = -inf)
-        m_used = mx;
-      }
-      if (j > 0 && __any_sync(0xffffffffu, need)) {
-        uint32_t o[32];
-#pragma unroll
-        for (int hlf = 0; hlf < 2; ++hlf) {
-          tmem_ld_32x32(tmem_O + lane_off + hlf * 32, o);
-          tmem_ld_wait();
-#pragma unroll
-          for (int c = 0; c < 32; ++c) o[c] = __float_as_uint(__uint_as_float(o[c]) * corr);
-          tmem_st_32x32(tmem_O + lane_off + hlf * 32, o);
-        }
-        tmem_st_wait();
-      }
-      lsum *= corr;
-      float psum = 0.f;
-#pragma unroll
-      for (int c8 = 0; c8 < 8; ++c8) {
-        uint32_t w[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const float p0 = ex2(__uint_as_float(r[8 * c8 + 2 * e]) - m_used);
-          const float p1 = ex2(__uint_as_float(r[8 * c8 + 2 * e + 1]) - m_used);
-          psum += p0 + p1;
-          w[e] = (uint32_t)__bfloat16_as_ushort(to16(p0, a.fp16)) | ((uint32_t)__bfloat16_as_ushort(to16(p1, a.fp16)) << 16);
-        }
-        *reinterpret_cast<uint4*>(prow + ((c8 ^ sw) << 4)) = make_uint4(w[0], w[1], w[2], w[3]);
-      }
-      lsum += psum;
-      fence_proxy_async();   // generic-proxy smem writes -> visible to the tensor core (async proxy)
-      tc_fence_before();
-      mbar_arrive(p_ready);
-    }
-    mbar_wait(o_done, 0);
-    tc_fence_after();
-    uint32_t o[64];
-    tmem_ld_32x32(tmem_O + lane_off, o);
-    tmem_ld_32x32(tmem_O + lane_off + 32, o + 32);
-    tmem_ld_wait();
-    if (qvalid) {
-      const float inv = 1.0f / lsum;
-      bf16* op = a.out + ((long long)b * T + tq) * a.ldo + hi * 64;
-#pragma unroll
-      for (int c8 = 0; c8 < 8; ++c8) {
-        uint32_t hw[4], lw[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          bf16 h0, l0, h1, l1;
-          split_bf16(__uint_as_float(o[8 * c8 + 2 * e]) * inv, h0, l0, a.fp16);
-          split_bf16(__uint_as_float(o[8 * c8 + 2 * e + 1]) * inv, h1, l1, a.fp16);
-          hw[e] = (uint32_t)__bfloat16_as_ushort(h0) | ((uint32_t)__bfloat16_as_ushort(h1) << 16);
-          lw[e] = (uint32_t)__bfloat16_as_ushort(l0) | ((uint32_t)__bfloat16_as_ushort(l1) << 16);
-        }
-        *reinterpret_cast<uint4*>(op + 8 * c8) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-        if (a.out_planes > 1) *reinterpret_cast<uint4*>(op + a.out_plane + 8 * c8) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
-      }
-    }
-    tc_fence_before();
-  }
-  __syncthreads();
-  if (warp == 5) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 128);
-  }
-}
-
-
 // ================================================================================================
-// v2: software-pipelined variant.  Differences from the kernel above:
+// v2: software-pipelined kernel (bf16 or fp16 operands; V row-major or transposed):
 //   * two S accumulators in TMEM: S_{j+1} = Q K_{j+1}^T is issued before the softmax of block j finishes, so the tensor
 //     pipe and the softmax warps overlap instead of alternating;
 //   * two P buffers and a 3-stage K/V ring to go with it;
@@ -532,7 +350,7 @@ __global__ void __launch_bounds__(A_THREADS, 2) attention_tc2_kernel(const __gri
 // The ones column that yields the softmax denominator rides on the two Vh passes (N = 80), so the denominator is
 // sum_k (Ph + Pl)[q,k] - exactly the P the numerator uses; the Vl pass runs with N = 64.
 // Shared memory: Q 2 x 16 KB, K / V rings 3 x (8 + 8) KB each, ones block 8 KB, P 2 x (16 + 16) KB = 200 KB: one CTA per SM.
-// Everything else (persistent head-major work list, S ping-pong in TMEM, lazy rescaling, gated bias from the table) is v2.
+// Everything else (persistent head-major work list, S ping-pong in TMEM, lazy rescaling, gated bias from the table) is as above.
 // ================================================================================================
 struct AttnMaps3 { CUtensorMap q[2], k[2], v[2]; };
 
@@ -797,14 +615,7 @@ __global__ void __launch_bounds__(A_THREADS, 1) attention_tc3_kernel(const __gri
   }
 }
 
-static bool attn_use_v1() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DZ_ATTN_V1"); v = (e && e[0] == '1') ? 1 : 0; }
-  return v == 1;
-}
-
 AttnPlan* attention_tc_plan_create(const AttnArgs& a, int B) {
-  if (attn_use_v1() && a.v != nullptr) return nullptr;   // the first-generation kernel only takes the transposed V
   AttnPlan* p = new AttnPlan();
   p->a = a;
   p->B = B;
@@ -846,9 +657,8 @@ AttnPlan* attention_tc_plan_create(const AttnArgs& a, int B) {
     uint32_t box[3] = {ABK, 64, 1};
     if (!make_tmap_bf16(&p->maps.vt, a.vt, 3, dims, str, box)) { delete p; return nullptr; }
   }
-  if (attn_use_v1()) p->smem = 1024 + 16384 + 2 * 8192 + 2 * 8192 + 16384 + 80 + sizeof(float) * (size_t)(2 * T - 1 + 64 + 8);
-  else p->smem = 1024 + 16384 + KV_STAGES * 8192 + (a.v != nullptr ? KV_STAGES * 8192 + 8192 : KV_STAGES * V_STAGE_BYTES) + 2 * 16384 + 128 +
-                 sizeof(float) * (size_t)(2 * T - 1 + 64 + 8);
+  p->smem = 1024 + 16384 + KV_STAGES * 8192 + (a.v != nullptr ? KV_STAGES * 8192 + 8192 : KV_STAGES * V_STAGE_BYTES) + 2 * 16384 + 128 +
+            sizeof(float) * (size_t)(2 * T - 1 + 64 + 8);
   return p;
 }
 void attention_tc_plan_destroy(AttnPlan* p) { delete p; }
@@ -870,10 +680,8 @@ cudaError_t attention_tc_plan_launch(const AttnPlan* p, cudaStream_t st) {
     return cudaGetLastError();
   }
   static size_t attr = 0;
-  const bool v1 = attn_use_v1();
   if (p->smem > attr) {
-    cudaError_t e = cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_tc2_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
+    cudaError_t e = cudaFuncSetAttribute(attention_tc2_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_tc2_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_tc2_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_tc2_kernel<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
@@ -881,25 +689,21 @@ cudaError_t attention_tc_plan_launch(const AttnPlan* p, cudaStream_t st) {
     attr = p->smem;
   }
   dim3 grid((p->a.T + ABQ - 1) / ABQ, p->a.nheads, p->B);
-  if (v1) {
-    attention_tc_kernel<<<grid, A_THREADS, p->smem, st>>>(p->maps, p->a);
-  } else {
-    static int slots = 0;
-    if (!slots) {
-      int dev = 0, sms = 148;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-      slots = 2 * sms;   // two resident CTAs per SM (launch bounds, 110 KB of shared memory and 256 TMEM columns each)
-    }
-    const long long items = (long long)grid.x * grid.y * grid.z;
-    const unsigned g = (unsigned)(items < slots ? items : slots);
-    const int variant = (p->a.fp16 ? 1 : 0) | (p->a.v != nullptr ? 2 : 0);
-    switch (variant) {
-      case 0: attention_tc2_kernel<0, 0><<<g, A_THREADS, p->smem, st>>>(p->maps, p->a, p->B); break;
-      case 1: attention_tc2_kernel<1, 0><<<g, A_THREADS, p->smem, st>>>(p->maps, p->a, p->B); break;
-      case 2: attention_tc2_kernel<0, 1><<<g, A_THREADS, p->smem, st>>>(p->maps, p->a, p->B); break;
-      default: attention_tc2_kernel<1, 1><<<g, A_THREADS, p->smem, st>>>(p->maps, p->a, p->B); break;
-    }
+  static int slots = 0;
+  if (!slots) {
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    slots = 2 * sms;   // two resident CTAs per SM (launch bounds, 110 KB of shared memory and 256 TMEM columns each)
+  }
+  const long long items = (long long)grid.x * grid.y * grid.z;
+  const unsigned g = (unsigned)(items < slots ? items : slots);
+  const int variant = (p->a.fp16 ? 1 : 0) | (p->a.v != nullptr ? 2 : 0);
+  switch (variant) {
+    case 0: attention_tc2_kernel<0, 0><<<g, A_THREADS, p->smem, st>>>(p->maps, p->a, p->B); break;
+    case 1: attention_tc2_kernel<1, 0><<<g, A_THREADS, p->smem, st>>>(p->maps, p->a, p->B); break;
+    case 2: attention_tc2_kernel<0, 1><<<g, A_THREADS, p->smem, st>>>(p->maps, p->a, p->B); break;
+    default: attention_tc2_kernel<1, 1><<<g, A_THREADS, p->smem, st>>>(p->maps, p->a, p->B); break;
   }
   return cudaGetLastError();
 }

@@ -14,7 +14,6 @@
 #include <string>
 #include <vector>
 
-#include <cstdlib>
 #include "../../include/diarizen_b200.h"
 #include "common.cuh"
 #include "emb_kernels.h"
@@ -263,8 +262,7 @@ static int emb_plan(dz_emb* s, int B, int N, int S, int T) {
       s->steps.push_back({nm, [d](cudaStream_t st) { return gemm_simt_launch(d, st); }, flops, 0.0});
       return;
     }
-    static const bool c3_off = [] { const char* e = getenv("DZ_CONV3_GENERIC"); return e && e[0] == '1'; }();
-    if (!c3_off && ks == 3 && stride == 1 && Cin == Cout && (Cin == 32 || Cin == 64) && P == 1 && s->npass == 1 && act == 3) {
+    if (ks == 3 && stride == 1 && Cin == Cout && (Cin == 32 || Cin == 64) && P == 1 && s->npass == 1 && act == 3) {
       // layer1 / layer2: resident weights + row-shifted A views instead of the generic implicit GEMM (conv3x3_c32.cu)
       Conv3Args c{};
       c.in = in.p; c.out = out.p; c.res = res ? res->p : nullptr; c.w = W.w.as<bf16>(); c.ldw = W.ldb; c.bias = W.bias.as<float>();
@@ -275,8 +273,7 @@ static int emb_plan(dz_emb* s, int B, int N, int S, int T) {
       s->steps.push_back({nm, [cp](cudaStream_t st) { return conv3x3_c32_plan_launch(cp, st); }, flops, 0.0});
       return;
     }
-    static const bool c128_off = [] { const char* e = getenv("DZ_CONV128_GENERIC"); return e && e[0] == '1'; }();
-    if (!c128_off && ks == 3 && stride == 1 && Cin == Cout && Cin == 128 && P == 1 && s->npass == 1 && act == 3) {
+    if (ks == 3 && stride == 1 && Cin == Cout && Cin == 128 && P == 1 && s->npass == 1 && act == 3) {
       // layer3: streamed weights, two output rows per tile, row-shifted A views (conv3x3_c128.cu)
       Conv3Args c{};
       c.in = in.p; c.out = out.p; c.res = res ? res->p : nullptr; c.w = W.w.as<bf16>(); c.ldw = W.ldb; c.bias = W.bias.as<float>();

@@ -3,114 +3,15 @@
 // 3x3 convolution (C_in = 1 stencil) and the masked statistics pooling (4 speaker masks per trunk output).
 // reference: pyannote-audio/pyannote/audio/models/embedding/wespeaker/__init__.py:80-103 (compute_fbank),
 //            wespeaker/resnet.py:358 (conv1 + bn1 + relu), resnet.py:49-66 + models/blocks/pooling.py:44-131 (TSTP).
-#include <cstdlib>
-
 #include "common.cuh"
 #include "emb_kernels.h"
 
 namespace dz {
 
 // ------------------------------------------------------------------------------------------------
-// K13 fbank: one warp per frame.  torchaudio.compliance.kaldi.fbank(num_mel_bins=80, frame 25 ms / 10 ms,
+// K13 fbank: torchaudio.compliance.kaldi.fbank(num_mel_bins=80, frame 25 ms / 10 ms,
 // dither 0, hamming, remove_dc_offset, preemphasis 0.97, round_to_power_of_two, use_power, use_log_fbank),
-// applied to waveform * 2^15.
-// ------------------------------------------------------------------------------------------------
-static constexpr int FB_WIN = 400, FB_HOP = 160, FB_NFFT = 512, FB_BINS = 257;
-
-__global__ void __launch_bounds__(256) fbank_kernel(FbankArgs a) {
-  extern __shared__ float2 smf[];
-  float2* tw = smf;                       // 256 twiddles
-  float2* bufs = smf + 256;               // 8 x 512 complex
-  __shared__ float win[FB_WIN];
-  for (int i = threadIdx.x; i < 256; i += blockDim.x) tw[i] = a.twiddle[i];
-  for (int i = threadIdx.x; i < FB_WIN; i += blockDim.x) win[i] = a.window[i];
-  __syncthreads();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int f = blockIdx.x * 8 + warp;
-  const int b = blockIdx.y;
-  if (f >= a.F) return;
-  float2* X = bufs + warp * FB_NFFT;
-  float* xr = reinterpret_cast<float*>(X);   // scratch for the raw frame (first 400 floats)
-  const float* src = a.wav + (long long)b * a.N + (long long)f * FB_HOP;
-  float s = 0.f;
-  for (int i = lane; i < FB_WIN; i += 32) {
-    const float v = src[i] * 32768.0f;
-    xr[i] = v;
-    s += v;
-  }
-  const float mean = warp_sum(s) / FB_WIN;
-  __syncwarp();
-  float y[13];
-#pragma unroll
-  for (int j = 0; j < 13; ++j) {
-    const int i = lane + 32 * j;
-    float v = 0.f;
-    if (i < FB_WIN) {
-      const float cur = xr[i] - mean;
-      const float prev = xr[i > 0 ? i - 1 : 0] - mean;
-      v = (cur - 0.97f * prev) * win[i];
-    }
-    y[j] = v;
-  }
-  __syncwarp();
-  // bit-reversed load of the (zero padded) real frame
-#pragma unroll
-  for (int j = 0; j < 16; ++j) {
-    const int i = lane + 32 * j;
-    const float v = (j < 13) ? y[j < 13 ? j : 0] : 0.f;
-    const int r = __brev((unsigned)i) >> 23;  // 9-bit reversal
-    X[r] = make_float2((i < FB_WIN) ? v : 0.f, 0.f);
-  }
-  __syncwarp();
-  // radix-2 decimation-in-time, 9 stages, 256 butterflies per stage, 8 per lane
-#pragma unroll 1
-  for (int st = 0; st < 9; ++st) {
-    const int half = 1 << st;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const int t = lane + 32 * j;           // butterfly index 0..255
-      const int k = t & (half - 1);
-      const int i0 = ((t >> st) << (st + 1)) + k;
-      const int i1 = i0 + half;
-      const float2 w = tw[k << (8 - st)];
-      const float2 u = X[i0], v = X[i1];
-      const float2 wv = make_float2(w.x * v.x - w.y * v.y, w.x * v.y + w.y * v.x);
-      X[i0] = make_float2(u.x + wv.x, u.y + wv.y);
-      X[i1] = make_float2(u.x - wv.x, u.y - wv.y);
-    }
-    __syncwarp();
-  }
-  // power spectrum into the (now free) upper half of the buffer is not possible in place: use registers
-  float pw[9];
-#pragma unroll
-  for (int j = 0; j < 9; ++j) {
-    const int k = lane + 32 * j;
-    float p = 0.f;
-    if (k < FB_BINS) { const float2 c = X[k]; p = c.x * c.x + c.y * c.y; }
-    pw[j] = p;
-  }
-  __syncwarp();
-  float* P = reinterpret_cast<float*>(X);
-#pragma unroll
-  for (int j = 0; j < 9; ++j) {
-    const int k = lane + 32 * j;
-    if (k < FB_BINS) P[k] = pw[j];
-  }
-  __syncwarp();
-  // mel-major output [b][mel][frame]: the consumers (mean over frames, 3x3 conv over (mel, frame)) walk along frames
-  float* dst = a.out + (long long)b * 80 * a.F + f;
-  for (int m = lane; m < 80; m += 32) {
-    const int ks = a.mel_range[2 * m], ke = a.mel_range[2 * m + 1];
-    const float* wrow = a.mel_w + m * FB_BINS;
-    float acc = 0.f;
-    for (int k = ks; k < ke; ++k) acc = fmaf(P[k], __ldg(wrow + k), acc);
-    dst[(long long)m * a.F] = logf(fmaxf(acc, 1.1920928955078125e-07f));
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// fbank, second generation (default; DZ_FBANK_V1=1 selects the kernel above).  Same arithmetic per sample up to the
-// FFT, which is reorganised around the register file instead of shared memory:
+// applied to waveform * 2^15.  The 512-point FFT is organised around the register file:
 //  * a warp transforms TWO frames at once (frame f -> real part, frame f + 1 -> imaginary part of one complex sequence;
 //    the spectra are separated afterwards as A[k] = (Z[k] + conj Z[N-k]) / 2, B[k] = (Z[k] - conj Z[N-k]) / 2i);
 //  * 512 = 8 x 8 x 8: every lane holds 16 complex points and runs two 8-point DFTs per step in registers; between the
@@ -119,6 +20,7 @@ __global__ void __launch_bounds__(256) fbank_kernel(FbankArgs a) {
 //    X = sum_n3 W8^{n3 k3} W512^{n3 (k1 + 8 k2)} sum_n2 W8^{n2 k2} W64^{n2 k1} sum_n1 W8^{n1 k1} x);
 //  * the per-lane twiddles of both steps are tabulated once per CTA; a CTA walks 64 frames.
 // ------------------------------------------------------------------------------------------------
+static constexpr int FB_WIN = 400, FB_HOP = 160, FB_NFFT = 512, FB_BINS = 257;
 static constexpr int FB2_S = 72;        // exchange row stride (== 8 mod 32)
 static constexpr int FB2_Z = 576;       // per-warp floats per component: 8 * 72 = 576 = 512 + 4 * 16 (padded spectrum)
 static constexpr int FB2_FRAMES = 64;   // frames per CTA
@@ -298,16 +200,9 @@ __global__ void __launch_bounds__(256, 3) fbank2_kernel(FbankArgs a) {
 }
 
 cudaError_t launch_fbank(const FbankArgs& a, int B, cudaStream_t st) {
-  static const bool v1 = [] { const char* e = getenv("DZ_FBANK_V1"); return e && e[0] == '1'; }();
-  if (!v1) {
-    dim3 grid2((a.F + FB2_FRAMES - 1) / FB2_FRAMES, B);
-    const size_t smem2 = sizeof(float) * (416 + 2 * 512 * 2 + 8 * 2 * FB2_Z);
-    fbank2_kernel<<<grid2, 256, smem2, st>>>(a);
-    return cudaGetLastError();
-  }
-  dim3 grid((a.F + 7) / 8, B);
-  const size_t smem = sizeof(float2) * (256 + 8 * FB_NFFT);
-  fbank_kernel<<<grid, 256, smem, st>>>(a);
+  dim3 grid((a.F + FB2_FRAMES - 1) / FB2_FRAMES, B);
+  const size_t smem = sizeof(float) * (416 + 2 * 512 * 2 + 8 * 2 * FB2_Z);
+  fbank2_kernel<<<grid, 256, smem, st>>>(a);
   return cudaGetLastError();
 }
 
@@ -380,7 +275,8 @@ __global__ void __launch_bounds__(256) emb_conv1_kernel(Conv1Args a) {
     }
   }
 }
-// Second generation (default; DZ_EMB_CONV1_V1=1 selects the kernel above).  One CTA per (window, mel) output row: the three
+// Row kernel, used whenever its three staged rows fit the default 48 KB of shared memory (F up to 4094 frames; the kernel
+// above takes longer inputs).  One CTA per (window, mel) output row: the three
 // mean-subtracted input rows are staged once in shared memory; a thread owns 8 of the 32 output channels, keeps their 72
 // weights (and the folded BatchNorm) in registers for the whole row and walks the frames, so the inner loop is 9 shared-memory
 // reads + 72 FMAs per (pixel, channel group) instead of one shared-memory weight read per FMA, there is no 64-bit division per
@@ -437,9 +333,8 @@ __global__ void __launch_bounds__(256, 2) emb_conv1_rows_kernel(Conv1Args a) {
   }
 }
 cudaError_t launch_emb_conv1(const Conv1Args& a, cudaStream_t st) {
-  static const bool v1 = [] { const char* e = getenv("DZ_EMB_CONV1_V1"); return e && e[0] == '1'; }();
   const size_t smem = sizeof(float) * 3 * (size_t)(a.F + 2);
-  if (!v1 && smem <= 48 * 1024) {
+  if (smem <= 48 * 1024) {
     emb_conv1_rows_kernel<<<a.B * 80, 256, smem, st>>>(a);
     return cudaGetLastError();
   }

@@ -17,7 +17,6 @@
 // This kernel replaces the cuBLAS/cuDNN calls behind nn.Linear / nn.Conv1d on the reference hot path
 // (reference: diarizen/models/module/wav2vec2/components.py:119 conv1d, :305-306 projection, :374 pos-conv,
 //  :455-480 q/k/v/out projections, :805-814 FFN; diarizen/models/module/conformer.py:116-214).
-#include <cstdlib>
 #include <mutex>
 #include <string>
 
@@ -903,8 +902,6 @@ static cudaError_t launch_bn_tma(const GemmPlan* p, cudaStream_t st) {
 // the same kind as the output (or none), and an activation after the residual only when it is ReLU (the one it applies
 // after the add).  Everything else takes the generic epilogue.
 static bool tma_epilogue_eligible(const GemmDesc& d) {
-  static const bool off = (getenv("DZ_GEMM_LEGACY_EPILOGUE") != nullptr);
-  if (off && d.ln_gamma == nullptr) return false;
   if (d.groups != 1 || d.out_t != nullptr) return false;
   if (d.act_after_res && d.act != 0 && d.act != 3) return false;
   const bool f = d.out_f32 != nullptr, h = d.out_bf != nullptr;
@@ -1029,9 +1026,8 @@ cudaError_t gemm_plan_launch(const GemmPlan* p, cudaStream_t st) {
       case 128: return launch_bn_tma<128>(p, st);
       case 256: {
         // deep ring when nothing is prefetched into the store patches and one 4 KB patch holds a span (single plane)
-        static const bool no_deep = (getenv("DZ_GEMM_NO_DEEP") != nullptr);
         const GemmDesc& d = p->d;
-        const bool deep = !no_deep && d.residual == nullptr && d.res16 == nullptr && !(p->epi_mode == 1 && d.out_planes > 1);
+        const bool deep = d.residual == nullptr && d.res16 == nullptr && !(p->epi_mode == 1 && d.out_planes > 1);
         return deep ? launch_bn_tma<256, 1>(p, st) : launch_bn_tma<256, 0>(p, st);
       }
     }

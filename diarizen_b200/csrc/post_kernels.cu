@@ -6,7 +6,6 @@
 // reference: diarizen/pipelines/inference.py:131-132, pyannote-audio/pyannote/audio/core/inference.py:543-666,
 //   pipelines/utils/diarization.py:122-157,193-239, pipelines/speaker_diarization.py:271-320,377-425,
 //   pipelines/clustering.py:159-173,404-418 (scipy linkage(method="centroid") on unit-norm embeddings).
-#include <cstdlib>
 #include <string>
 
 #include "../../include/diarizen_b200.h"
@@ -377,8 +376,8 @@ DZ_DEVINL void block_argmin2(ArgMin& a, ArgMin& b, ArgMin* sc) {
   }
 }
 
-// The default merge loop (DZ_LINKAGE_V1=1 selects the kernel above): the same arithmetic, the same (distance, index)
-// order for the closest pair, organised for one SM's latency and float64 budget:
+// The default merge loop for N < 65535 (its slot indices are 16-bit; the kernel above takes larger N): the same arithmetic,
+// the same (distance, index) order for the closest pair, organised for one SM's latency and float64 budget:
 //  * state (nnd, nn, size, the compact list of live slots and its inverse) in shared memory as 8 + 4 x 2 bytes per slot
 //    (N <= ~14 000; beyond that the same code runs on the global workspace); initial neighbours from linkage_nn_init_kernel;
 //  * only LIVE slots are visited: the update loop and the row scans walk the compact list, so a step costs O(live), not O(N)
@@ -593,9 +592,7 @@ int dz_linkage_centroid_variant(double* dist_dev, int N, double* z_dev, void* wo
   int* nn = (int*)w; w += (size_t)N * 4;
   char* rest = w;                                          // 8 N bytes: v1's size + todo, or the lazy kernel's 16-bit state
   unsigned long long* counters = (unsigned long long*)(rest + (size_t)N * 8);   // in the 256-byte tail: [0] = row rescans of the last call
-  static const bool env_v1 = [] { const char* e = getenv("DZ_LINKAGE_V1"); return e && e[0] == '1'; }();
-  const bool v1 = variant == 1 || (variant == 0 && env_v1);
-  if (!v1 && N < 65535) {
+  if (variant != 1 && N < 65535) {
     const size_t smem = (size_t)N * (8 + 4 * 2);
     const bool in_smem = smem <= 220 * 1024 && variant != 2;
     // 512 threads x 16 loads in flight: ~10 % faster than 1024 x 8 on every data set tried (cheaper barriers, no spills)

@@ -16,7 +16,6 @@
 #include <string>
 #include <vector>
 
-#include <cstdlib>
 #include "../../include/diarizen_b200.h"
 #include "common.cuh"
 #include "gemm.h"
@@ -436,10 +435,9 @@ static int plan_impl(dz_seg* s, int B, int N) {
       p.step("conv0_moments", [s, B, N, T0, mom](cudaStream_t st) { return launch_conv0_moments(s->cur_wav, B, N, T0, mom, st); });
       p.step("conv0_gn_coef", [=](cudaStream_t st) { return launch_conv0_gn_coef(mom, w0, g0, b0, B, C0, T0, coef, st); });
     }
-    // conv0_tc.cu (tcgen05) is the default since it matched the oracle on the s80 configurations at the benchmarked sizes
-    // (tests/test_bench_config_gpu.py); DZ_CONV0_SIMT=1 selects the CUDA-core kernel for A/B runs
-    static const bool c0_want_tc = [] { const char* e = getenv("DZ_CONV0_SIMT"); return !(e && e[0] == '1'); }();
-    const bool c0_tc = c0_want_tc && s->gemm_impl == 0 && conv0_tc_eligible(c);
+    // conv0_tc.cu (tcgen05) runs whenever the tensor-core GEMMs do and it takes the shape (it matches the oracle on the s80
+    // configurations at the benchmarked sizes, tests/test_bench_config_gpu.py); otherwise the CUDA-core kernel runs
+    const bool c0_tc = s->gemm_impl == 0 && conv0_tc_eligible(c);
     p.step("conv0", [s, c, B, large, c0_tc](cudaStream_t st) {
              Conv0Args cc = c; cc.wav = s->cur_wav;
              return c0_tc ? launch_conv0_tc(cc, B, large, st) : launch_conv0(cc, B, large, st);
@@ -457,8 +455,7 @@ static int plan_impl(dz_seg* s, int B, int N) {
     d.a_bstride = (long long)Tl[l - 1] * Cp[l - 1]; d.a_rows_alloc = Tl[l];
     d.b = W.w.p; d.b_plane = W.plane; d.ldb = W.ldb; d.b_gstride = W.gstride;
     const bool last = (l == 6);
-    static const bool ln_unfused = [] { const char* e = getenv("DZ_CONV_LN_UNFUSED"); return e && e[0] == '1'; }();
-    if (large && !last && !ln_unfused && s->gemm_impl == 0 && W.N <= 256) {
+    if (large && !last && s->gemm_impl == 0 && W.N <= 256) {
       // conv -> LayerNorm(channels) -> GELU in one launch: the accumulator tile holds whole rows (N <= 256), so the
       // normalisation happens on the TMEM row before the 16-bit planes are stored (no fp32 round trip through HBM)
       d.ln_gamma = s->conv_gamma[l].as<float>(); d.ln_beta = s->conv_beta[l].as<float>(); d.ln_eps = 1e-5f; d.act = 1;
@@ -528,8 +525,7 @@ static int plan_impl(dz_seg* s, int B, int N) {
     d.bias = W.bias.as<float>(); d.act = 1; d.group_cols = Dg;
     d.residual = xres; d.res_bstride = (long long)T * Dp; d.ldr = Dp;
     d.out_f32 = xres; d.of_bstride = (long long)T * Dp; d.ldo = Dp;
-    static const bool pc_generic = [] { const char* e = getenv("DZ_POSCONV_GENERIC"); return e && e[0] == '1'; }();
-    if (!pc_generic && s->npass == 1 && s->gemm_impl == 0 && Dg % 4 == 0) {
+    if (s->npass == 1 && s->gemm_impl == 0 && Dg % 4 == 0) {
       PosConvArgs pa{};
       pa.stage = stage.p; pa.stage_rows = PCR; pa.stage_ld = PCW; pa.w = W.w.as<bf16>(); pa.ldw = W.ldb; pa.w_gstride = W.gstride;
       pa.bias = W.bias.as<float>(); pa.x = xres; pa.ldx = Dp; pa.B = B; pa.T = T; pa.Dg = Dg; pa.fp16 = FP;

@@ -3,7 +3,6 @@
 // the conformer depthwise convolution, the classifier / log-softmax / powerset head.
 // Reference call sites are cited per kernel.
 #include <cstdint>
-#include <cstdlib>
 
 #include "common.cuh"
 #include "seg_kernels.h"
@@ -609,10 +608,9 @@ static void launch_ln_fast_nv(const LnArgs& a, unsigned grid, cudaStream_t st) {
 }
 
 cudaError_t launch_layernorm(const LnArgs& a, cudaStream_t st) {
-  static const bool generic = [] { const char* e = getenv("DZ_LN_GENERIC"); return e && e[0] == '1'; }();
   // rows must be padded to a multiple of 4 floats; with the layer mix (always D-wide, D % 4 == 0) or a ragged C the
   // chunk straddling C is masked in registers
-  const bool fast = !generic && (a.ldx % 4) == 0 && a.ldx >= ((a.C + 3) & ~3) && (a.y_f32 == nullptr || (a.ldy % 4 == 0 && a.ldy >= ((a.C + 3) & ~3))) &&
+  const bool fast = (a.ldx % 4) == 0 && a.ldx >= ((a.C + 3) & ~3) && (a.y_f32 == nullptr || (a.ldy % 4 == 0 && a.ldy >= ((a.C + 3) & ~3))) &&
                     (a.mix == nullptr || (a.C % 4) == 0);
   if (fast) {
     if (a.C > 1024) return cudaErrorInvalidValue;
@@ -707,8 +705,7 @@ __global__ void __launch_bounds__(256) regroup_to_bf16_vec8_kernel(const float* 
 }
 cudaError_t launch_regroup(const float* x, long long rows, int C, int ldx, int seq_len, int seq_rows_out, int row_off,
                            int gin, int gout, bf16* out, long long out_plane, int ldo, int planes, int fp16, cudaStream_t st) {
-  static const bool scalar = [] { const char* e = getenv("DZ_REGROUP_SCALAR"); return e && e[0] == '1'; }();
-  if (!scalar && C % 8 == 0 && gin % 8 == 0 && gout % 8 == 0 && ldx % 4 == 0 && ldo % 8 == 0 && out_plane % 8 == 0 &&
+  if (C % 8 == 0 && gin % 8 == 0 && gout % 8 == 0 && ldx % 4 == 0 && ldo % 8 == 0 && out_plane % 8 == 0 &&
       (((uintptr_t)x) & 15) == 0 && (((uintptr_t)out) & 15) == 0) {
     const int grid = (int)min((long long)148 * 8, (rows + 7) / 8);
     regroup_to_bf16_vec8_kernel<<<grid, 256, 0, st>>>(x, rows, C, ldx, seq_len, seq_rows_out, row_off, gin, gout, out, out_plane,
@@ -962,9 +959,10 @@ __global__ void __launch_bounds__(256) glu_dwconv_kernel(DwArgs a) {
     }
   }
 }
-// v2 (default; DZ_DWCONV_V1=1 selects the kernel above): same accumulation order per output, fast-intrinsic sigmoids (ncu of
-// the IEEE-division version: 264 instructions per output, most of them the two sigmoids); 64 frames per CTA (halo overhead 1.47x instead of 1.94x) and four outputs per thread in
-// flight, which share every shared-memory load (0.27 LDS per FMA instead of 1) and break the dependent FMA chain.
+// v2, used whenever its shared memory fits in 200 KB (the kernel above takes wider heads): same accumulation order per
+// output, fast-intrinsic sigmoids (ncu of the IEEE-division version: 264 instructions per output, most of them the two
+// sigmoids); 64 frames per CTA (halo overhead 1.47x instead of 1.94x) and four outputs per thread in flight, which share
+// every shared-memory load (0.27 LDS per FMA instead of 1) and break the dependent FMA chain.
 static constexpr int DW2_TT = 64;
 template <int KS>   // KS > 0: kernel size known at compile time (31 in every shipped configuration) - no per-tap predicates
 __global__ void __launch_bounds__(256) glu_dwconv_v2_kernel(DwArgs a) {
@@ -1030,21 +1028,18 @@ __global__ void __launch_bounds__(256) glu_dwconv_v2_kernel(DwArgs a) {
 
 cudaError_t launch_glu_dwconv(const DwArgs& a, int B, cudaStream_t st) {
   if (a.ksize > 32) return cudaErrorInvalidValue;
-  static const bool v2 = [] { const char* e = getenv("DZ_DWCONV_V1"); return !(e && e[0] == '1'); }();
-  if (v2) {
-    const size_t smem2 = sizeof(float) * (size_t)(DW2_TT + a.ksize - 1) * a.A;
-    if (smem2 <= 200 * 1024) {
-      static size_t attr2 = 0;
-      if (smem2 > 48 * 1024 && smem2 > attr2) {
-        cudaFuncSetAttribute(glu_dwconv_v2_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-        cudaFuncSetAttribute(glu_dwconv_v2_kernel<31>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-        attr2 = smem2;
-      }
-      dim3 grid2((a.T + DW2_TT - 1) / DW2_TT, B);
-      if (a.ksize == 31) glu_dwconv_v2_kernel<31><<<grid2, 256, smem2, st>>>(a);
-      else glu_dwconv_v2_kernel<0><<<grid2, 256, smem2, st>>>(a);
-      return cudaGetLastError();
+  const size_t smem2 = sizeof(float) * (size_t)(DW2_TT + a.ksize - 1) * a.A;
+  if (smem2 <= 200 * 1024) {
+    static size_t attr2 = 0;
+    if (smem2 > 48 * 1024 && smem2 > attr2) {
+      cudaFuncSetAttribute(glu_dwconv_v2_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
+      cudaFuncSetAttribute(glu_dwconv_v2_kernel<31>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
+      attr2 = smem2;
     }
+    dim3 grid2((a.T + DW2_TT - 1) / DW2_TT, B);
+    if (a.ksize == 31) glu_dwconv_v2_kernel<31><<<grid2, 256, smem2, st>>>(a);
+    else glu_dwconv_v2_kernel<0><<<grid2, 256, smem2, st>>>(a);
+    return cudaGetLastError();
   }
   const size_t smem = sizeof(float) * (size_t)(DW_TT + a.ksize - 1) * a.A;
   static size_t attr = 0;

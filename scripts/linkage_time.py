@@ -1,5 +1,6 @@
 """Times dz_pdist + dz_linkage_centroid on clustered unit-norm rows (the shape of the AHC input in the pipeline bench).
-usage: python scripts/linkage_time.py N [check]   (env DZ_LINKAGE_V1 / DZ_LINKAGE_NT / DZ_LINKAGE_EXP select variants)"""
+usage: python scripts/linkage_time.py N [check]   (env LINK_VARIANT is the variant argument of dz_linkage_centroid_variant:
+0 default, 1 first-generation loop, 2 lazy loop with its state in global memory)"""
 import ctypes as C
 import sys
 import time
@@ -16,6 +17,7 @@ check = len(sys.argv) > 2
 L = _lib.lib()
 g = np.random.default_rng(5)
 kind = os.environ.get("LINK_DATA", "hard")
+variant = int(os.environ.get("LINK_VARIANT", "0"))
 cent = g.standard_normal((6, 256))
 noise = {"hard": 0.35, "easy": 0.05, "uniform": 10.0}[kind]
 x = cent[g.integers(0, 6, N)] + noise * g.standard_normal((N, 256))
@@ -32,7 +34,8 @@ for it in range(4):
     ev[0].record()
     _lib.check(L.dz_pdist(C.c_void_p(xd.data_ptr()), N, 256, C.c_void_p(dist.data_ptr()), st))
     ev[1].record()
-    _lib.check(L.dz_linkage_centroid(C.c_void_p(dist.data_ptr()), N, C.c_void_p(Z.data_ptr()), C.c_void_p(ws.data_ptr()), st))
+    _lib.check(L.dz_linkage_centroid_variant(C.c_void_p(dist.data_ptr()), N, C.c_void_p(Z.data_ptr()), C.c_void_p(ws.data_ptr()), st,
+                                             variant))
     ev[2].record()
     torch.cuda.synchronize()
     res.append((ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2])))
